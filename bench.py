@@ -51,6 +51,9 @@ def parse_args():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-predict", action="store_true")
     ap.add_argument("--watchdog-seconds", type=int, default=1500, help="hard exit if the whole run takes longer (a hung collective must not eat the box)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed boosting rounds (the rounds/sec metric), write the model "
+                    "they trained (every tree array, float32 / float64) as DIR/<name>.npy, so two builds can be compared on identical "
+                    "seeded inputs; the e2e and predict sections are not dumped, and --impl reference does not take it")
     return ap.parse_args()
 
 
@@ -249,6 +252,17 @@ def model_hash(be, bst):
     return h.hexdigest()[:16], int(len(m["tree_info"]))
 
 
+def dump_outputs(be, bst, out_dir):
+    """The booster as the timed rounds left it: tree arrays (ints as float64, exact) and the float32 node values."""
+    os.makedirs(out_dir, exist_ok=True)
+    m = be.booster_export_model(bst.handle)
+    for k in ("tree_offset", "tree_info", "left", "right", "parent", "split_index", "split_bin", "default_left", "split_cond",
+              "base_weight", "loss_chg", "sum_hess"):
+        a = np.asarray(m[k])
+        np.save(os.path.join(out_dir, k + ".npy"), a.astype(np.float32 if a.dtype == np.float32 else np.float64))
+    np.save(os.path.join(out_dir, "base_score.npy"), np.array([m["base_score"]], np.float64))
+
+
 def predict_section(xgb, be, device, peak):
     """BASELINE config 5 (second half of the metric: predict rows/sec): a 1M-row x 28 `text/csv` request body through the
     serving path the container's default handler takes -- csv_to_dmatrix (encoder.py:35-52, here parsed on the device) then
@@ -312,6 +326,8 @@ def main():
         wd.daemon = True
         wd.start()
     if a.impl == "reference":
+        if a.dump_outputs:
+            sys.exit("bench.py: --dump-outputs applies to the CUDA path (--impl b200) only")
         run_reference(a)
         return
     import torch
@@ -367,6 +383,8 @@ def main():
     clk = clocks.stop() if rank == 0 else None
     ms = max_over_ranks(ms)
     mhash, mtrees = model_hash(be, bst)           # after warm-up + timed rounds: the same trees at every N
+    if a.dump_outputs and rank == 0:
+        dump_outputs(be, bst, a.dump_outputs)
     # per-kernel CUDA-event timing of the histogram launches: the timed region above replays a CUDA graph per tree, so the
     # events bracket the same launches issued directly for PROFILE_ROUNDS further rounds right after it (same state, same data)
     be.booster_set_profile(bst.handle, True)

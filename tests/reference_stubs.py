@@ -1,15 +1,9 @@
-"""Import stubs so the reference container's own modules (read-only at /root/reference, only present in the build
-container) can be imported in this image: the third-party packages below are not installed here and are not on the
-hot path.  Nothing of the reference is copied; its modules run unchanged on top of our `xgboost` replacement."""
+"""Import stubs so the container's own modules (from a checkout of aws/sagemaker-xgboost-container, used by
+tests/golden/make_container_goldens.py to record golden vectors) import without the third-party packages below, which are
+not on the hot path.  Nothing of the container is copied; its modules run unchanged on top of our `xgboost` replacement."""
 import os
 import sys
 import types
-
-REFERENCE_SRC = "/root/reference/src"
-
-
-def reference_available():
-    return os.path.isdir(os.path.join(REFERENCE_SRC, "sagemaker_xgboost_container"))
 
 
 def _mod(name, **attrs):
@@ -19,8 +13,9 @@ def _mod(name, **attrs):
     return m
 
 
-def install(xgb_pkg):
-    """Alias our package as `xgboost`, stub the absent third-party modules, put the reference sources on sys.path."""
+def install(xgb_pkg, checkout):
+    """Alias our package as `xgboost`, stub the absent third-party modules, put the container sources of `checkout` on sys.path."""
+    src = os.path.join(checkout, "src")
     xgb_pkg.install_as_xgboost()
     if "xgboost.dask" not in sys.modules:
         d = _mod("xgboost.dask", DaskDMatrix=type("DaskDMatrix", (), {}), train=None)
@@ -51,15 +46,15 @@ def install(xgb_pkg):
         _mod("botocore", exceptions=be)
         sm = _mod("sagemaker", fw_utils=_mod("sagemaker.fw_utils"), utils=_mod("sagemaker.utils"))
         del sm
-    if REFERENCE_SRC not in sys.path:
-        sys.path.insert(0, REFERENCE_SRC)
+    if src not in sys.path:
+        sys.path.insert(0, src)
     # algorithm_mode/__init__.py only pre-loads the serving model (and drags in flask/gunicorn): register the package
     # without executing that __init__, so that algorithm_mode.train / serve_utils themselves are imported unchanged.
     name = "sagemaker_xgboost_container.algorithm_mode"
     if name not in sys.modules:
         import sagemaker_xgboost_container  # noqa: F401
         pkg = types.ModuleType(name)
-        pkg.__path__ = [os.path.join(REFERENCE_SRC, "sagemaker_xgboost_container", "algorithm_mode")]
+        pkg.__path__ = [os.path.join(src, "sagemaker_xgboost_container", "algorithm_mode")]
         pkg.__package__ = name
         sys.modules[name] = pkg
         sys.modules["sagemaker_xgboost_container"].algorithm_mode = pkg
