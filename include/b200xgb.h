@@ -172,6 +172,17 @@ XGB_DLL int XGB200BuildHistogramEx(BoosterHandle handle, DMatrixHandle dmat, con
                              const char** out_kernel);
 /* mean device time (CUDA events) of the predictor kernel alone over `repeats` launches on `dmat` */
 XGB_DLL int XGB200BoosterPredictKernelMs(BoosterHandle handle, DMatrixHandle dmat, int repeats, float* out_ms);
+/* The predictor's launch plan as JSON: {"route": "tiled" | "thread_per_row", "kernel": ..., "pitch": floats per staged row,
+ * "absent_features": bool (the matrix is narrower than the model), "node_budget": bytes, "smem_limit": bytes,
+ * "chunks": [{"tree_lo", "tree_hi", "rows", "threads", "head", "smem"}, ...]}, chunks in tree order covering
+ * [tree_begin, tree_end) on the tiled route.  XGB200PredictPlan is host code only (no device needed): node_counts holds the
+ * node slots of trees tree_begin .. tree_end-1.  XGB200BoosterPredictPlan reports the plan XGBoosterPredictFromDMatrix runs
+ * on `dmat` for the iteration range [iteration_begin, iteration_end) (0, 0 = all rounds), from the model's device slot sizes.
+ * *out_json is a thread-local buffer (the handle's, for the Booster form), valid until the next string-returning call. */
+XGB_DLL int XGB200PredictPlan(int data_features, int model_features, const int64_t* node_counts, int tree_begin, int tree_end,
+                              int children_adjacent, const char** out_json);
+XGB_DLL int XGB200BoosterPredictPlan(BoosterHandle handle, DMatrixHandle dmat, int iteration_begin, int iteration_end,
+                                     const char** out_json);
 /* raw margins of the prediction cache the trainer keeps for `dmat` (n x num_class), brought up to date first */
 XGB_DLL int XGB200BoosterGetCachedMargin(BoosterHandle handle, DMatrixHandle dmat, float* out);
 /* CUDA-event stopwatch on the engine's stream: Start records an event, Stop records another, waits, returns ms */

@@ -406,6 +406,21 @@ class CudaBackend:
         self._check(self.lib.XGB200BoosterPredictKernelMs(bh, dh, C.c_int(repeats), C.byref(ms)))
         return float(ms.value)
 
+    def predict_plan(self, data_features, model_features, node_counts, tree_begin=0, children_adjacent=True):
+        """The predictor's launch plan for trees [tree_begin, tree_begin + len(node_counts)) (host code, no device)."""
+        counts = np.ascontiguousarray(node_counts, np.int64)
+        out = C.c_char_p()
+        self._check(self.lib.XGB200PredictPlan(C.c_int(data_features), C.c_int(model_features), counts.ctypes.data_as(C.POINTER(C.c_int64)),
+                                               C.c_int(tree_begin), C.c_int(tree_begin + len(counts)), C.c_int(1 if children_adjacent else 0),
+                                               C.byref(out)))
+        return json.loads(out.value.decode())
+
+    def booster_predict_plan(self, bh, dh, iteration_range=(0, 0)):
+        """The plan XGBoosterPredictFromDMatrix runs for `dh` over `iteration_range`."""
+        out = C.c_char_p()
+        self._check(self.lib.XGB200BoosterPredictPlan(bh, dh, C.c_int(int(iteration_range[0])), C.c_int(int(iteration_range[1])), C.byref(out)))
+        return json.loads(out.value.decode())
+
     def booster_cached_margin(self, bh, dh, K):
         n = self.dmatrix_num_row(dh)
         out = np.zeros((n, K), np.float32)

@@ -646,6 +646,14 @@ void Booster::upload_model() {
   }
 }
 
+PredictArgs Booster::predict_args(const DMatrix* dm, int tree_begin, int tree_end) const {
+  PredictArgs pa{}; pa.X = dm->X.p; pa.n = dm->n; pa.F = dm->F; pa.F_model = num_feature_;
+  pa.nodes = d_nodes.p; pa.tree_offset = d_tree_offset.p; pa.tree_info = d_tree_info.p;
+  pa.tree_begin = tree_begin; pa.tree_end = tree_end; pa.K = param_.num_class; pa.margin = nullptr; pa.leaf = nullptr;
+  pa.h_tree_offset = h_tree_offset.data(); pa.has_nan = dm->has_missing ? 1 : 0; pa.children_adjacent = children_adjacent_ ? 1 : 0;
+  return pa;
+}
+
 PredCache& Booster::cache_for(DMatrix* dm) {
   PredCache& c = caches_[dm->uid];
   const int K = param_.num_class;
@@ -668,9 +676,7 @@ void Booster::bring_cache_up_to_date(DMatrix* dm, PredCache& c) {
   }
   if (c.trees_applied < nt) {
     upload_model();
-    PredictArgs pa{}; pa.X = dm->X.p; pa.n = dm->n; pa.F = dm->F; pa.nodes = d_nodes.p; pa.tree_offset = d_tree_offset.p; pa.tree_info = d_tree_info.p;
-    pa.tree_begin = c.trees_applied; pa.tree_end = nt; pa.K = K; pa.margin = c.margin.p; pa.leaf = nullptr;
-    pa.h_tree_offset = h_tree_offset.data(); pa.has_nan = dm->has_missing ? 1 : 0; pa.children_adjacent = children_adjacent_ ? 1 : 0;
+    PredictArgs pa = predict_args(dm, c.trees_applied, nt); pa.margin = c.margin.p;
     launch_predict(pa, s);
     c.trees_applied = nt;
   }
@@ -1083,16 +1089,12 @@ void Booster::predict(DMatrix* dm, int type, bool training, int iter_begin, int 
   const int rounds = (int)trees_.size() / K;
   if (iter_end == 0) iter_end = rounds;
   B200_CHECK(iter_begin >= 0 && iter_begin <= iter_end && iter_end <= rounds, "Invalid iteration range: [" + std::to_string(iter_begin) + ", " + std::to_string(iter_end) + ") for a model with " + std::to_string(rounds) + " rounds");
-  if (num_feature_ > 0 && !trees_.empty())
-    B200_CHECK(dm->F <= num_feature_ || true, "feature count mismatch");
   B200_CHECK(type == 0 || type == 1 || type == 2 || type == 6, "predict type " + std::to_string(type) + " (approximate contributions / interactions) is not implemented on the B200 path");
   if (type == 2) { predict_contribs(dm, iter_begin * K, iter_end * K, out, shape); return; }
   upload_model();
   const int tb = iter_begin * K, te = iter_end * K;
   const int64_t n = dm->n;
-  PredictArgs pa{}; pa.X = dm->X.p; pa.n = n; pa.F = dm->F; pa.nodes = d_nodes.p; pa.tree_offset = d_tree_offset.p; pa.tree_info = d_tree_info.p;
-  pa.tree_begin = tb; pa.tree_end = te; pa.K = K;
-  pa.h_tree_offset = h_tree_offset.data(); pa.has_nan = dm->has_missing ? 1 : 0; pa.children_adjacent = children_adjacent_ ? 1 : 0;
+  PredictArgs pa = predict_args(dm, tb, te);          // a feature the matrix lacks (column >= dm->F) is missing on every route
   if (type == 6) {
     const int nt = te - tb;
     DevBuf<int>& leaf = pred_leaf_; leaf.ensure((size_t)n * std::max(nt, 1));
@@ -1243,9 +1245,7 @@ float Booster::debug_predict_kernel_ms(DMatrix* dm, int repeats) {
   upload_model();
   const int K = param_.num_class;
   pred_margin_.ensure((size_t)dm->n * K);
-  PredictArgs pa{}; pa.X = dm->X.p; pa.n = dm->n; pa.F = dm->F; pa.nodes = d_nodes.p; pa.tree_offset = d_tree_offset.p; pa.tree_info = d_tree_info.p;
-  pa.tree_begin = 0; pa.tree_end = (int)trees_.size(); pa.K = K; pa.margin = pred_margin_.p; pa.leaf = nullptr;
-  pa.h_tree_offset = h_tree_offset.data(); pa.has_nan = dm->has_missing ? 1 : 0; pa.children_adjacent = children_adjacent_ ? 1 : 0;
+  PredictArgs pa = predict_args(dm, 0, (int)trees_.size()); pa.margin = pred_margin_.p;
   cudaEvent_t e0, e1; CUDA_OK(cudaEventCreate(&e0)); CUDA_OK(cudaEventCreate(&e1));
   float total = 0.f;
   for (int r = 0; r < std::max(1, repeats); ++r) {
@@ -1258,6 +1258,19 @@ float Booster::debug_predict_kernel_ms(DMatrix* dm, int repeats) {
   }
   cudaEventDestroy(e0); cudaEventDestroy(e1);
   return total / std::max(1, repeats);
+}
+
+std::string Booster::predict_plan(DMatrix* dm, int iter_begin, int iter_end) {
+  configure();
+  const int K = param_.num_class;
+  const int rounds = (int)trees_.size() / K;
+  if (iter_end == 0) iter_end = rounds;
+  B200_CHECK(iter_begin >= 0 && iter_begin <= iter_end && iter_end <= rounds, "Invalid iteration range: [" + std::to_string(iter_begin) + ", " + std::to_string(iter_end) + ") for a model with " + std::to_string(rounds) + " rounds");
+  upload_model();                                  // device slot sizes: trained trees keep their fixed-capacity slots
+  const int tb = iter_begin * K, te = iter_end * K;
+  std::vector<int64_t> counts(te - tb);
+  for (int t = tb; t < te; ++t) counts[t - tb] = h_tree_offset[t + 1] - h_tree_offset[t];
+  return predict_plan_json(plan_predict(dm->F, num_feature_, counts.data(), tb, te, children_adjacent_));
 }
 
 void Booster::cached_margin(DMatrix* dm, std::vector<float>* out) {

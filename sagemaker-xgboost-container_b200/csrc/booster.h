@@ -112,6 +112,7 @@ class Booster {
   void sync_model();                              // materialise pending trees on the host
   void cached_margin(DMatrix* dm, std::vector<float>* out);   // the trainer's prediction cache for dm
   float debug_predict_kernel_ms(DMatrix* dm, int repeats);
+  std::string predict_plan(DMatrix* dm, int iter_begin, int iter_end);   // JSON of the plan predict() would run on dm
   const std::vector<HostTree>& trees() { sync_model(); return trees_; }
   const std::vector<int>& tree_info() const { return tree_info_; }
   float base_score() const { return base_score_; }
@@ -158,6 +159,7 @@ class Booster {
   float base_margin() const;
   void estimate_base_score(DMatrix* dtrain);
   void upload_model();
+  PredictArgs predict_args(const DMatrix* dm, int tree_begin, int tree_end) const;   // margin / leaf left null
   PredCache& cache_for(DMatrix* dm);
   void bring_cache_up_to_date(DMatrix* dm, PredCache& c);
   void append_device_tree(int class_id, size_t device_offset, int max_nodes, PendingTree pt);

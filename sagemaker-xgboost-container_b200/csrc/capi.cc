@@ -519,6 +519,21 @@ int XGB200BoosterPredictKernelMs(BoosterHandle handle, DMatrixHandle dmat, int r
   *out_ms = BST(handle)->debug_predict_kernel_ms(DM(dmat), repeats);
   API_END();
 }
+int XGB200PredictPlan(int data_features, int model_features, const int64_t* node_counts, int tree_begin, int tree_end,
+                      int children_adjacent, const char** out_json) {
+  API_BEGIN();
+  B200_CHECK(out_json != nullptr && tree_begin >= 0 && tree_end >= tree_begin && (node_counts != nullptr || tree_end == tree_begin),
+             "XGB200PredictPlan: bad argument");
+  g_ret_str = predict_plan_json(plan_predict(data_features, model_features, node_counts, tree_begin, tree_end, children_adjacent != 0));
+  *out_json = g_ret_str.c_str();
+  API_END();
+}
+int XGB200BoosterPredictPlan(BoosterHandle handle, DMatrixHandle dmat, int iteration_begin, int iteration_end, const char** out_json) {
+  API_BEGIN();
+  BoosterBox* box = static_cast<BoosterBox*>(handle);
+  box->ret_str = BST(handle)->predict_plan(DM(dmat), iteration_begin, iteration_end); *out_json = box->ret_str.c_str();
+  API_END();
+}
 int XGB200BoosterGetCachedMargin(BoosterHandle handle, DMatrixHandle dmat, float* out) {
   API_BEGIN();
   std::vector<float> v;

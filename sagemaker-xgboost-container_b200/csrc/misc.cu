@@ -250,6 +250,10 @@ __global__ void __launch_bounds__(1024) predict_tiled_kernel(PredictArgs a, int 
   }
   float* s_x = reinterpret_cast<float*>(s_nodes + s_total);
   const int F = a.F, K = a.K, nt_all = a.tree_end - a.tree_begin;
+  if (F < a.F_model) {                                                          // features the matrix lacks are missing; the tile
+    const int w = a.F_model - F;                                                // loads below never overwrite these slots
+    for (int i = threadIdx.x; i < rows_per_tile * w; i += blockDim.x) { const int r = i / w; s_x[r * pitch + F + (i - r * w)] = __int_as_float(0x7fc00000); }
+  }
   for (int64_t tile = blockIdx.x; tile < num_tiles; tile += gridDim.x) {
     const int64_t r0 = tile * rows_per_tile;
     const int rows = (int)((a.n - r0 < rows_per_tile) ? a.n - r0 : rows_per_tile);
@@ -409,60 +413,86 @@ void launch_replace_missing(float* X, int64_t count, float missing, cudaStream_t
   if (count == 0) return;
   replace_missing_kernel<<<grid_for(count), 256, 0, s>>>(X, count, missing); ++g_kernel_launches; CUDA_OK(cudaGetLastError());
 }
-// host-side plan of the tiled predictor: trees are cut into chunks that fit in shared memory next to a row tile
+// Plan of the tiled predictor: trees are cut, in order, into chunks whose packed nodes fit in shared memory next to a tile of
+// at least 32 rows.  Anything the tiled kernel cannot hold takes the thread-per-row kernel.
+PredictPlan plan_predict(int F, int F_model, const int64_t* node_counts, int tree_begin, int tree_end, bool children_adjacent) {
+  PredictPlan p;
+  const int width = std::max(F, F_model);                          // a narrower matrix is staged at the model's width, NaN-padded
+  p.pitch = width | 1;                                             // odd pitch: threads of a warp (rows) hit different banks for the same feature
+  p.absent_features = F < F_model;
+  const size_t min_tile = (size_t)p.pitch * 4 * 32;
+  if (!(width <= 32767 && children_adjacent) || min_tile + 64 * 1024 > kPredictSmem) return p;   // 15-bit feature field
+  p.node_budget = 96 * 1024;                                       // bytes of packed nodes per chunk
+  auto offsets = [](int trees) { return ((size_t)(trees + 1) * 4 + 15) & ~(size_t)15; };
+  auto fits = [&](int trees, size_t bytes) { return bytes <= p.node_budget && offsets(trees) + bytes + min_tile <= kPredictSmem; };
+  int lo = tree_begin;
+  while (lo < tree_end) {
+    int hi = lo; size_t bytes = 0;
+    while (hi < tree_end) {
+      const int64_t nn = node_counts[hi - tree_begin];
+      if (nn > 65534) { p.chunks.clear(); return p; }              // the packed node keeps a 16-bit child index
+      if (!fits(hi - lo + 1, bytes + (size_t)nn * 8)) {
+        if (hi == lo) { p.chunks.clear(); return p; }              // a tree too large for any chunk
+        break;
+      }
+      bytes += (size_t)nn * 8; ++hi;
+    }
+    PredictChunk c;
+    c.tree_lo = lo; c.tree_hi = hi;
+    c.head = offsets(hi - lo) + bytes;
+    int rows = (int)((kPredictSmem - c.head) / ((size_t)p.pitch * 4));
+    rows = rows > 1024 ? 1024 : (rows / 32) * 32;
+    c.threads = rows >= 1024 ? 1024 : (rows >= 512 ? 512 : 256);
+    c.rows = rows > c.threads ? c.threads : rows;                  // one row per thread and tile
+    c.smem = c.head + (size_t)c.rows * p.pitch * 4;
+    p.chunks.push_back(c);
+    lo = hi;
+  }
+  p.tiled = true;
+  return p;
+}
+
+std::string predict_plan_json(const PredictPlan& p) {
+  std::string s = std::string("{\"route\":\"") + (p.tiled ? "tiled" : "thread_per_row") + "\",\"kernel\":\"" +
+                  (p.tiled ? "predict_tiled_kernel" : "predict_kernel") + "\",\"pitch\":" + std::to_string(p.pitch) +
+                  ",\"absent_features\":" + (p.absent_features ? "true" : "false") + ",\"node_budget\":" + std::to_string(p.node_budget) +
+                  ",\"smem_limit\":" + std::to_string(kPredictSmem) + ",\"chunks\":[";
+  for (size_t i = 0; i < p.chunks.size(); ++i) {
+    const PredictChunk& c = p.chunks[i];
+    s += std::string(i ? "," : "") + "{\"tree_lo\":" + std::to_string(c.tree_lo) + ",\"tree_hi\":" + std::to_string(c.tree_hi) +
+         ",\"rows\":" + std::to_string(c.rows) + ",\"threads\":" + std::to_string(c.threads) + ",\"head\":" + std::to_string(c.head) +
+         ",\"smem\":" + std::to_string(c.smem) + "}";
+  }
+  return s + "]}";
+}
+
 void launch_predict(const PredictArgs& a, cudaStream_t s) {
   if (a.n == 0 || a.tree_end <= a.tree_begin) return;
-  static const bool legacy = getenv("B200XGB_PREDICT_LEGACY") != nullptr;
-  const bool ok = !legacy && a.h_tree_offset != nullptr && a.F <= 32767 && a.children_adjacent;
-  const int pitch = a.F | 1;                                       // odd pitch: threads of a warp (rows) hit different banks for the same feature
-  const size_t kSmem = 220 * 1024;
-  if (ok && (size_t)pitch * 4 * 32 + 64 * 1024 <= kSmem) {
-    static bool attr = false;
-    if (!attr) {
-      CUDA_OK(cudaFuncSetAttribute(predict_tiled_kernel<false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kSmem));
-      CUDA_OK(cudaFuncSetAttribute(predict_tiled_kernel<true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kSmem));
-      CUDA_OK(cudaFuncSetAttribute(predict_tiled_kernel<false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kSmem));
-      CUDA_OK(cudaFuncSetAttribute(predict_tiled_kernel<true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kSmem));
-      attr = true;
-    }
-    const size_t node_budget = 96 * 1024;                          // bytes of packed nodes per chunk
-    int lo = a.tree_begin;
-    bool fits = true;
-    std::vector<std::pair<int, int>> chunks;
-    while (lo < a.tree_end) {
-      int hi = lo; size_t bytes = 0;
-      while (hi < a.tree_end) {
-        const int64_t nn = a.h_tree_offset[hi + 1] - a.h_tree_offset[hi];
-        if (nn > 65534) { fits = false; break; }
-        if (bytes + (size_t)nn * 8 > node_budget && hi > lo) break;
-        if ((size_t)nn * 8 > node_budget) { fits = false; break; }
-        bytes += (size_t)nn * 8; ++hi;
-      }
-      if (!fits) break;
-      chunks.emplace_back(lo, hi); lo = hi;
-    }
-    if (fits) {
-      for (auto& ch : chunks) {
-        size_t node_bytes = 0;
-        for (int t = ch.first; t < ch.second; ++t) node_bytes += (size_t)(a.h_tree_offset[t + 1] - a.h_tree_offset[t]) * 8;
-        const size_t head = (((size_t)(ch.second - ch.first + 1) * 4 + 15) & ~(size_t)15) + node_bytes;
-        int rows = (int)((kSmem - head) / ((size_t)pitch * 4));
-        rows = rows > 1024 ? 1024 : (rows / 32) * 32;
-        const int threads = rows >= 1024 ? 1024 : (rows >= 512 ? 512 : 256);
-        if (rows > threads) rows = threads;                        // one row per thread and tile
-        const int64_t tiles = (a.n + rows - 1) / rows;
-        const int grid = (int)std::min<int64_t>(tiles, 148 * (threads == 1024 ? 1 : 2048 / threads));
-        const size_t smem = head + (size_t)rows * pitch * 4;
-        if (a.leaf) { if (a.has_nan) predict_tiled_kernel<true, true><<<grid, threads, smem, s>>>(a, ch.first, ch.second, pitch, rows, tiles);
-                      else predict_tiled_kernel<false, true><<<grid, threads, smem, s>>>(a, ch.first, ch.second, pitch, rows, tiles); }
-        else { if (a.has_nan) predict_tiled_kernel<true, false><<<grid, threads, smem, s>>>(a, ch.first, ch.second, pitch, rows, tiles);
-               else predict_tiled_kernel<false, false><<<grid, threads, smem, s>>>(a, ch.first, ch.second, pitch, rows, tiles); }
-        ++g_kernel_launches; CUDA_OK(cudaGetLastError());
-      }
-      return;
-    }
+  std::vector<int64_t> counts(a.tree_end - a.tree_begin);
+  for (int t = a.tree_begin; t < a.tree_end; ++t) counts[t - a.tree_begin] = a.h_tree_offset[t + 1] - a.h_tree_offset[t];
+  const PredictPlan p = plan_predict(a.F, a.F_model, counts.data(), a.tree_begin, a.tree_end, a.children_adjacent != 0);
+  if (!p.tiled) {
+    predict_kernel<<<(unsigned)((a.n + 255) / 256), 256, 0, s>>>(a); ++g_kernel_launches; CUDA_OK(cudaGetLastError());
+    return;
   }
-  predict_kernel<<<(unsigned)((a.n + 255) / 256), 256, 0, s>>>(a); ++g_kernel_launches; CUDA_OK(cudaGetLastError());
+  static bool attr = false;
+  if (!attr) {
+    CUDA_OK(cudaFuncSetAttribute(predict_tiled_kernel<false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kPredictSmem));
+    CUDA_OK(cudaFuncSetAttribute(predict_tiled_kernel<true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kPredictSmem));
+    CUDA_OK(cudaFuncSetAttribute(predict_tiled_kernel<false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kPredictSmem));
+    CUDA_OK(cudaFuncSetAttribute(predict_tiled_kernel<true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kPredictSmem));
+    attr = true;
+  }
+  const bool nan = a.has_nan || p.absent_features;
+  for (const PredictChunk& c : p.chunks) {
+    const int64_t tiles = (a.n + c.rows - 1) / c.rows;
+    const int grid = (int)std::min<int64_t>(tiles, 148 * (c.threads == 1024 ? 1 : 2048 / c.threads));
+    if (a.leaf) { if (nan) predict_tiled_kernel<true, true><<<grid, c.threads, c.smem, s>>>(a, c.tree_lo, c.tree_hi, p.pitch, c.rows, tiles);
+                  else predict_tiled_kernel<false, true><<<grid, c.threads, c.smem, s>>>(a, c.tree_lo, c.tree_hi, p.pitch, c.rows, tiles); }
+    else { if (nan) predict_tiled_kernel<true, false><<<grid, c.threads, c.smem, s>>>(a, c.tree_lo, c.tree_hi, p.pitch, c.rows, tiles);
+           else predict_tiled_kernel<false, false><<<grid, c.threads, c.smem, s>>>(a, c.tree_lo, c.tree_hi, p.pitch, c.rows, tiles); }
+    ++g_kernel_launches; CUDA_OK(cudaGetLastError());
+  }
 }
 void launch_transform(float* m, int64_t n, int K, int objective, float* out_class, cudaStream_t s) {
   if (n == 0) return;

@@ -23,14 +23,30 @@ struct DevNode { float cond; int left; int right; unsigned fidx_dl; };   // 16 B
 
 struct PredictArgs {
   const float* X; int64_t n; int F;
+  int F_model;              // features of the model; a matrix narrower than that lacks features F..F_model-1 (missing)
   const DevNode* nodes; const int64_t* tree_offset; const int* tree_info;
   int tree_begin, tree_end, K;
   float* margin;            // n x K, pre-initialised with the base margin; may be nullptr
   int* leaf;                // n x (tree_end - tree_begin); may be nullptr
-  const int64_t* h_tree_offset;   // host copy of tree_offset (plans the shared-memory tree chunks); nullptr = thread-per-row kernel
+  const int64_t* h_tree_offset;   // host copy of tree_offset (plans the shared-memory tree chunks)
   int has_nan;              // the matrix contains missing values
   int children_adjacent;    // right child == left child + 1 in every tree (true for every tree this engine trains)
 };
+
+// Host-side plan of one predictor call: either the thread-per-row kernel, or the tiled kernel run once per chunk of trees,
+// each chunk's packed nodes staged in shared memory next to a tile of `rows` rows at `pitch` floats per row.
+struct PredictChunk { int tree_lo, tree_hi, rows, threads; size_t head, smem; };   // head: tree offsets + packed nodes (bytes)
+struct PredictPlan {
+  bool tiled = false;
+  int pitch = 0;            // floats per staged row: max(F, F_model) | 1
+  bool absent_features = false;    // F < F_model: the staged slots F..F_model-1 hold NaN, so the NaN-aware variant runs
+  size_t node_budget = 0;   // bytes of packed nodes one chunk may hold
+  std::vector<PredictChunk> chunks;
+};
+constexpr size_t kPredictSmem = 220 * 1024;       // dynamic shared memory of the tiled predictor (B200: 227 KB per block)
+// node_counts[i] = device node slots of tree tree_begin + i; pure host code, touches no device
+PredictPlan plan_predict(int F, int F_model, const int64_t* node_counts, int tree_begin, int tree_end, bool children_adjacent);
+std::string predict_plan_json(const PredictPlan& p);
 
 enum Metric : int { kMetricRmse = 0, kMetricMae = 1, kMetricLogloss = 2, kMetricError = 3, kMetricMerror = 4, kMetricMlogloss = 5,
                     kMetricAuc = 6, kMetricMse = 7, kMetricRmsle = 8, kMetricMape = 9, kMetricMphe = 10, kMetricPoissonNll = 11,
